@@ -680,7 +680,12 @@ def main():
                          "the factor bytes drop from n(p1+p2) to p1^2+p2^2 per side (not the headline configuration)")
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-decode', action='store_true', help='skip the one-token decode legs (quick runs)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps write what the last timed step returned (the NLL of its sample, float32) to '
+                         'DIR/nll.npy; the inputs are fixed by seeds, so two builds can be compared output for output')
     a = ap.parse_args()
+    if a.dump_outputs and (a.impl != 'ours' or a.parallelism != 'dp'):
+        ap.error('--dump-outputs covers the timed data-parallel path (--impl ours --parallelism dp)')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     structure = 'blocked butterflies' if a.incoh == 'blocked' else 'Kronecker butterflies (pre_proj_extra 1): NOT the headline structure'
@@ -818,7 +823,8 @@ def main():
         e0.record()
         nll = torch.zeros((), device=dev)
         for i in range(a.warmup, total):
-            nll += step_fn(ids_dev[i])
+            last = step_fn(ids_dev[i])
+            nll += last
         if world > 1:
             dist.all_reduce(nll)
         e1.record()
@@ -826,6 +832,10 @@ def main():
         clk.mark_end()
         if profiling:
             torch.cuda.profiler.stop()
+    if a.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        np.save(os.path.join(a.dump_outputs, 'nll.npy'), last.float().cpu().numpy())
     with torch.no_grad():
         ms = max_over_ranks(e0.elapsed_time(e1))
         launches = lib.quip_launch_count() - launches0       # eager launches; a replayed graph is counted below

@@ -1,15 +1,15 @@
-"""Golden layer at a Llama-2-7B layer shape (4096 x 4096), quantized by the LIVE reference (build container only).
+"""Golden 1024 x 1024 layer quantized by the LIVE reference (build container only).
 
-Run:  python -m oracle.gen_golden_big [--method ldlq|nearest] [--n 4096 --k 4096]
+Run:  python -m oracle.gen_golden_big [--method ldlq|nearest] [--n 1024 --k 1024]
 
-The small golden layers (oracle/gen_golden.py) never exceed K = 640, so every GPU parity case built on them keeps the
-tcgen05 kernel on one tile per CTA.  This fixture is a whole q_proj-sized Linear through the reference's own flow
-(`Balance.preproc` with --pre_gptqH --pre_rescale --pre_proj, method.py:139-193; `fasterquant`, bal.py:21-48;
-`postproc`, method.py:195-214), so that the multi-tile persistent path, the 64 x 64 butterflies and the one-kernel
-sides are checked against the reference's own dense fp16 output `F.linear(x, W_ref)`.
+The small golden layers (oracle/gen_golden.py) never exceed K = 640.  This fixture is a whole Linear through the
+reference's own flow (`Balance.preproc` with --pre_gptqH --pre_rescale --pre_proj, method.py:139-193; `fasterquant`,
+bal.py:21-48; `postproc`, method.py:195-214), so that the multi-tile persistent path (its 16 tokens replicated to
+thousands), the 32 x 32 butterflies and the one-kernel sides are checked against the reference's own dense fp16 output
+`F.linear(x, W_ref)`.  1024 x 1024 keeps the file under 1 MB; a 4096 x 4096 layer needs 8 MB of codes and factors.
 
 To stay small the file keeps what the packer needs (codes as 2-bit planes, grid parameters, scaleWH, butterfly factors
-and permutations) plus a 16-token x / y_ref slice and eight rows of W_ref -- not W_ref itself (32 MiB).
+and permutations) plus a 16-token x / y_ref slice and eight rows of W_ref -- not W_ref itself.
 """
 import argparse
 import contextlib
@@ -38,10 +38,10 @@ def unpack2(packed):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--method', default='ldlq')
-    ap.add_argument('--n', type=int, default=4096)
-    ap.add_argument('--k', type=int, default=4096)
+    ap.add_argument('--n', type=int, default=1024)
+    ap.add_argument('--k', type=int, default=1024)
     ap.add_argument('--tokens', type=int, default=2048)
-    ap.add_argument('--name', default='big_4096')
+    ap.add_argument('--name', default='big_1024')
     a = ap.parse_args()
     mods = import_reference()
     quant, method, bal, _ = mods

@@ -56,8 +56,15 @@ def main(mods):
     ppl = float(buf.getvalue().strip().splitlines()[-1])
 
     out = dict(config=np.array(repr(TINY_OPT)), test_ids=test_ids.numpy(), ppl=np.float64(ppl))
-    for k, v in model.state_dict().items():
-        out['sd/' + k] = v.numpy()
+    sd = model.state_dict()
+    assert torch.equal(sd['lm_head.weight'], sd['model.decoder.embed_tokens.weight'])
+    for k, v in sd.items():
+        if k != 'lm_head.weight':                   # tied to the embedding: stored once, which keeps each file under 1 MB
+            out['sd/' + k] = v.numpy()
+    path = os.path.join(OUT, 'tiny_opt_2bit_incoh.npz')
+    np.savez_compressed(path, **out)
+    print('wrote', os.path.relpath(path, ROOT), f'{os.path.getsize(path)/1024:.0f} KiB', 'reference ppl', ppl)
+    out = {}
     names = []
     for lid, parts in cap.records.items():
         name = layers_by_id[lid]
@@ -76,7 +83,6 @@ def main(mods):
             out[p + side + '_p_in'] = b.p_in.numpy()
             out[p + side + '_p_out'] = b.p_out.numpy()
     out['names'] = np.array(names)
-    path = os.path.join(OUT, 'tiny_opt_2bit_incoh.npz')
+    path = os.path.join(OUT, 'tiny_opt_2bit_incoh_parts.npz')
     np.savez_compressed(path, **out)
-    print('wrote', os.path.relpath(path, ROOT), f'{os.path.getsize(path)/1024:.0f} KiB', 'reference ppl', ppl,
-          'layers', len(names))
+    print('wrote', os.path.relpath(path, ROOT), f'{os.path.getsize(path)/1024:.0f} KiB', 'layers', len(names))

@@ -9,7 +9,7 @@ Two checkers, both built from data the CUDA path does not share with them beyond
   * `reference_dense_weight(parts)`: the dense fp16 weight the reference leaves behind after `postproc`
     (method.py:195-214): W_ref = fp16( fp16(U^T Qhat V) / scaleWH ), Qhat the fp16 grid values; the reference's effective
     forward is then F.linear(x, W_ref, bias) (bal.py:44-45, opt.py:263-264).  Pinned against the live reference by
-    tests/golden/layer_big_4096.npz.
+    tests/golden/layer_big_1024.npz.
 
 Neither is a fallback: QuantLinear.forward raises without the CUDA library.
 """

@@ -80,10 +80,12 @@ def load_tiny_opt():
     from transformers import OPTConfig
     from quip_b200.capture import Butterfly, LayerParts
     from quip_b200.opt import get_opt
-    z = np.load(os.path.join(GOLDEN, 'tiny_opt_2bit_incoh.npz'))
-    cfg = OPTConfig(**ast.literal_eval(str(z['config'])))
+    m = np.load(os.path.join(GOLDEN, 'tiny_opt_2bit_incoh.npz'))
+    z = np.load(os.path.join(GOLDEN, 'tiny_opt_2bit_incoh_parts.npz'))
+    cfg = OPTConfig(**ast.literal_eval(str(m['config'])))
     model = get_opt(cfg)
-    sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith('sd/')}
+    sd = {k[3:]: torch.from_numpy(m[k]) for k in m.files if k.startswith('sd/')}
+    sd['lm_head.weight'] = sd['model.decoder.embed_tokens.weight']      # tied in OPT: stored once
     model.load_state_dict(sd)
     parts = {}
     for name in [str(n) for n in z['names']]:
@@ -97,11 +99,11 @@ def load_tiny_opt():
                                  scales=torch.from_numpy(z[p + 'scales']), zeros=torch.from_numpy(z[p + 'zeros']),
                                  bias=torch.from_numpy(z[p + 'bias']) if (p + 'bias') in z.files else None,
                                  scaleWH=torch.from_numpy(z[p + 'scaleWH']), U=bf('U', N), V=bf('V', K))
-    return model, parts, torch.from_numpy(z['test_ids']), float(z['ppl'])
+    return model, parts, torch.from_numpy(m['test_ids']), float(m['ppl'])
 
 
-def load_big_layer(name='big_4096'):
-    """Golden 4096 x 4096 layer quantized by the live reference (oracle/gen_golden_big.py) -> (LayerParts, npz)."""
+def load_big_layer(name='big_1024'):
+    """Golden 1024 x 1024 layer quantized by the live reference (oracle/gen_golden_big.py) -> (LayerParts, npz)."""
     import numpy as np
     import torch
     from quip_b200.capture import Butterfly, LayerParts

@@ -1,5 +1,5 @@
 """CPU: the dense-weight restatement (quip_b200/selfcheck.reference_dense_weight, method.py:195-214) pinned against a
-4096 x 4096 layer quantized by the live reference (tests/golden/layer_big_4096.npz, oracle/gen_golden_big.py)."""
+1024 x 1024 layer quantized by the live reference (tests/golden/layer_big_1024.npz, oracle/gen_golden_big.py)."""
 import torch
 
 from conftest import load_big_layer
@@ -32,7 +32,7 @@ def test_big_layer_packs_with_bit_exact_codes():
 
 def test_fp32_restatement_agrees_with_the_reference_outputs_on_the_cpu():
     """quip_b200/selfcheck.restated_forward (the checker bench.py and the GPU tests use) against the live reference's y_ref of
-    the golden layers and of the 4096 x 4096 layer: it is an independent, correct statement of the layer."""
+    the golden layers and of the 1024 x 1024 layer: it is an independent, correct statement of the layer."""
     import numpy as np
     from conftest import LAYER_NAMES, load_layer, parts_to_torch
     from quip_b200 import quant as Q

@@ -7,8 +7,9 @@ Here those launches are compared with a float64 contraction of the unpacked code
 rounding), checked for run-to-run determinism, and whole QuantLinear forwards at the same shapes are compared with
   * the fp32 restatement of the pipeline (quip_b200/selfcheck.restated_forward),
   * the reference's own dense path F.linear(x, W_ref), W_ref = fp16(fp16(U^T Q V)/s) (method.py:195-214), restated in
-    quip_b200/selfcheck.reference_dense_weight and pinned to the live reference by tests/golden/layer_big_4096.npz,
-  * the live reference's y_ref of that golden layer, replicated to 2048 tokens so it runs through the tcgen05 route.
+    quip_b200/selfcheck.reference_dense_weight and pinned to the live reference by tests/golden/layer_big_1024.npz,
+  * the live reference's y_ref of that golden layer, replicated to 2048 and 10240 tokens so it runs through the tcgen05
+    route, at 10240 tokens on 320 tiles (every persistent CTA walks several).
 Tolerance for whole layers: 1e-3 relative (north_star), norm-wise.
 """
 import json
@@ -117,10 +118,11 @@ def test_kronecker_layers_at_bench_shapes(K, N):
         assert torch.equal(y, ql(x[:M]))
 
 
-def test_golden_4096_layer_from_the_live_reference():
-    """tests/golden/layer_big_4096.npz: a q_proj-sized Linear quantized by the reference's own Balance flow (ldlq, 2 bits,
-    --incoh_processing).  Its 16-token y_ref through every token-count route, including 2048 tokens (the 16 rows
-    replicated 128 times, so the multi-tile tcgen05 path is compared with the live reference's own output)."""
+def test_golden_1024_layer_from_the_live_reference():
+    """tests/golden/layer_big_1024.npz: a 1024 x 1024 Linear quantized by the reference's own Balance flow (ldlq, 2 bits,
+    --incoh_processing).  Its 16-token y_ref through every token-count route, including 2048 and 10240 tokens (the 16 rows
+    replicated 128 and 640 times; 10240 tokens are 8 x 40 tiles on 148 persistent CTAs, so the multi-tile tcgen05 path is
+    compared with the live reference's own output)."""
     from quip_b200 import quant as Q
     from quip_b200.incoherence import plan_side
     from quip_b200.selfcheck import reference_dense_weight, rel_err
@@ -133,23 +135,23 @@ def test_golden_4096_layer_from_the_live_reference():
     assert torch.equal(ql.codes().cpu(), tp.codes[uo][:, vo])                  # integer codes bit-exact
     x = torch.from_numpy(z['x']).cuda()
     y_ref = torch.from_numpy(z['y_ref']).cuda()
-    for reps in (1, 3, 128):                                                    # 16, 48 and 2048 tokens
+    for reps in (1, 3, 128, 640):                                               # 16, 48, 2048 and 10240 tokens
         y = ql(x.repeat(reps, 1))
         err = rel_err(y, y_ref.repeat(reps, 1))
-        _report('golden_big_4096', M=16 * reps, rel_err_vs_reference=err)
+        _report('golden_big_1024', M=16 * reps, rel_err_vs_reference=err)
         assert err < 1e-3, (reps, err)
         if reps > 1:
             assert torch.equal(y[:16], y[-16:])                                # same rows, whatever tile they land in
     for M in (1, 5):
         err = rel_err(ql(x[:M]), y_ref[:M])
-        _report('golden_big_4096', M=M, rel_err_vs_reference=err)
+        _report('golden_big_1024', M=M, rel_err_vs_reference=err)
         assert err < 1e-3, (M, err)
-    # fresh activations at 2048 tokens against the dense weight restatement (pinned by tests/test_big_golden.py)
+    # fresh activations at 10240 tokens against the dense weight restatement (pinned by tests/test_big_golden.py)
     W_ref = reference_dense_weight(tp, 'cuda')
     assert rel_err(W_ref[:8].float().cpu(), torch.from_numpy(z['wref_rows']).float()) < 1e-4
-    xr = _inputs(2048, K, 7)
+    xr = _inputs(10240, K, 7)
     err = rel_err(ql(xr), torch.nn.functional.linear(xr, W_ref))
-    _report('golden_big_4096', M=2048, fresh_inputs=True, rel_err_vs_reference=err)
+    _report('golden_big_1024', M=10240, fresh_inputs=True, rel_err_vs_reference=err)
     assert err < 1e-3, err
 
 
