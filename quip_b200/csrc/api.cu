@@ -7,6 +7,9 @@
 #include <stdarg.h>
 #include <string.h>
 
+#include <map>
+#include <mutex>
+#include <tuple>
 #include <vector>
 
 #include "common.cuh"
@@ -23,58 +26,51 @@ void set_error(const char* fmt, ...) {
   va_end(ap);
 }
 
-// implemented in qgemm_skinny.cu / qgemm_tc.cu
-int qgemm_skinny(const QuipLinearDesc* d, const __half* x, const __half* bias, __half* z, int M, int ksplit,
-                 float* part, int* counters, cudaStream_t s);
-int skinny_pick_ksplit(int N, int K, int rows_per_cta, int M);
-size_t skinny_workspace_bytes(int N, int M, int ksplit);
-int qgemv(const QuipLinearDesc* d, const __half* x, const __half* bias, __half* z, int M, cudaStream_t s);
-bool qgemv_fits(int K, int M, int bits);
-int qgemm_tc(const QuipLinearDesc* d, const __half* x, const float* xsum, const __half* bias, __half* z, int M,
-             cudaStream_t s);
-
-extern int g_gather_rows, g_pass_min_tiles, g_fewtok;   // rot.cu
-extern int g_fewtok_max_m;                               // rot_fewtok.cu: token count up to which the few-token kernels run (8)
-bool side_fused_ok(const QuipSide* sd, int n);               // rot_side.cu
-int side_fused(const QuipSide* sd, const __half* in, __half* out, int64_t M, const int32_t* in_idx, const float* in_scale,
-               const int32_t* out_idx, const __half* out_bias, float* xsum, cudaStream_t s);
-bool pass_fewtok_ok(const QuipPass* ps, int64_t M, int n);   // rot_fewtok.cu
-int pass_fewtok(const QuipPass* ps, const __half* in, __half* out, int64_t M, int n, const int32_t* in_idx,
-                const float* in_scale, const int32_t* out_inv, const __half* out_bias, cudaStream_t s);
-extern int g_gv_rbc, g_gv_persist, g_gv_int, g_gv_tma, g_gv_cw, g_gv_stream;  // qgemv.cu
-bool side_fewtok_ok(const QuipSide* sd, int n, int64_t M);   // rot_side_fewtok.cu: both passes of a side in one launch, M <= 8
-int side_fewtok(const QuipSide* sd, const __half* in, __half* out, int64_t M, int n, const int32_t* in_idx,
-                const float* in_scale, const int32_t* out_inv, const __half* out_bias, cudaStream_t s);
-
 // tuning knobs (quip_config)
 static int g_side_fused = 1;     // many tokens: a whole side (gather + both passes [+ row sums]) in one kernel when the blocks allow
-static int g_pdl = 1;            // few-token kernels: programmatic dependent launch (weights prefetched under the previous kernel)
+int g_pdl = 1;                   // few-token kernels: programmatic dependent launch (weights prefetched under the previous kernel)
 static int g_use_gemv = 1;       // few-token contractions: whole-K qgemv kernel (0: the split-K kernel)
 static int g_sk_ksplit = 0;      // split-K kernel: cap on the number of K splits (0: the heuristic of skinny_pick_ksplit)
 static int g_side_fewtok = 0;    // <= 8 tokens: both passes of a side in ONE launch (rot_side_fewtok.cu), 3 launches per linear.
                                  // Correct on every shape but measured SLOWER than two pass launches (every CTA stages the whole
                                  // token vector): an ablation, off by default (profiles/README.md)
 
-// Launch with the programmatic-stream-serialization attribute: the kernel may start while its predecessor in
-// the stream drains; everything it does before griddepcontrol.wait must be independent of that predecessor.
-int launch_pdl(const void* kern, dim3 grid, dim3 block, size_t smem, cudaStream_t s, void** args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = g_pdl ? 1 : 0;
-  cudaError_t e = cudaLaunchKernelExC(&cfg, kern, args);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    set_error("kernel launch failed: %s", cudaGetErrorString(e));
-    return QUIP_ERR_CUDA;
-  }
-  return QUIP_OK;
+// ---- launch plumbing (common.cuh: launch) ----
+// The attribute and the occupancy query cost more host time than a decode kernel runs: both are cached.
+static std::mutex g_launch_mu;
+static std::map<std::pair<const void*, int>, size_t> g_smem_limit;                   // (kernel, device) -> bytes set
+static std::map<std::tuple<const void*, int, int, size_t>, int> g_occupancy;         // (kernel, device, threads, smem)
+static std::map<int, int> g_sms;                                                      // device -> SM count
+
+cudaError_t raise_smem_limit(const void* kern, size_t smem) {
+  if (smem == 0) return cudaSuccess;
+  int dev = 0;
+  if (cudaError_t e = cudaGetDevice(&dev)) return e;
+  std::lock_guard<std::mutex> lock(g_launch_mu);
+  size_t& set = g_smem_limit[{kern, dev}];
+  if (smem <= set) return cudaSuccess;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e == cudaSuccess) set = smem;
+  return e;
+}
+
+int num_sms() {
+  int dev = 0, n = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) return 148;
+  std::lock_guard<std::mutex> lock(g_launch_mu);
+  int& sms = g_sms[dev];
+  if (!sms) sms = cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess ? n : 148;
+  return sms;
+}
+
+// 1 when the query fails: the launch that follows reports the error
+int blocks_per_sm(const void* kern, int threads, size_t smem) {
+  int dev = 0, n = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || raise_smem_limit(kern, smem) != cudaSuccess) return 1;
+  std::lock_guard<std::mutex> lock(g_launch_mu);
+  int& occ = g_occupancy[{kern, dev, threads, smem}];
+  if (!occ) occ = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, threads, smem) == cudaSuccess && n > 1 ? n : 1;
+  return occ;
 }
 
 constexpr size_t WS_HEADER = 16 * 1024;     // split-K arrival counters; must be zero on first use, left zero

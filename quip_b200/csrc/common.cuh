@@ -5,7 +5,9 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <algorithm>
 #include <atomic>
+#include <utility>
 
 #include "../../include/quip_b200.h"
 
@@ -13,7 +15,6 @@ namespace quip {
 
 // ---- error plumbing (thread-local message, C ABI returns codes) -------------
 void set_error(const char* fmt, ...);
-extern std::atomic<int64_t> g_launches;
 
 #define QUIP_CHECK_ARG(cond, ...)            \
   do {                                       \
@@ -33,17 +34,76 @@ extern std::atomic<int64_t> g_launches;
     }                                                                                    \
   } while (0)
 
-// call right after a <<<>>> launch
-#define QUIP_LAUNCHED(name)                                                                   \
-  do {                                                                                        \
-    quip::g_launches.fetch_add(1, std::memory_order_relaxed);                                 \
-    cudaError_t _e = cudaPeekAtLastError();                                                   \
-    if (_e != cudaSuccess) {                                                                  \
-      cudaGetLastError();                                                                     \
-      quip::set_error("launch of %s failed: %s", name, cudaGetErrorString(_e));               \
-      return QUIP_ERR_CUDA;                                                                   \
-    }                                                                                         \
-  } while (0)
+// ---- kernel launches (api.cu) -----------------------------------------------------
+extern std::atomic<int64_t> g_launches;   // quip_launch_count
+extern int g_pdl;                         // quip_config("pdl")
+
+// Raise kern's max-dynamic-shared-memory attribute on the current device to smem, once per (kernel, device) and size;
+// the attribute is never lowered.
+cudaError_t raise_smem_limit(const void* kern, size_t smem);
+int num_sms();                                                     // of the current device
+int blocks_per_sm(const void* kern, int threads, size_t smem);     // occupancy (>= 1), cached per kernel, device and shape
+
+// Every kernel of the library starts here: kern<<<grid, block, smem, s>>>(args...), the shared-memory opt-in included,
+// counted in quip_launch_count.  The arguments convert to the kernel's parameter types as in a call.  With pdl (and
+// quip_config("pdl") on) the kernel may start while its predecessor in the stream drains (programmatic dependent
+// launch); everything it does before griddepcontrol.wait must then be independent of that predecessor.
+template <class... P, class... A>
+int launch(const char* name, void (*kern)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool pdl,
+           A&&... args) {
+  cudaError_t e = raise_smem_limit((const void*)kern, smem);
+  if (e == cudaSuccess) {
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cfg.attrs = attr;
+    cfg.numAttrs = pdl && g_pdl ? 1 : 0;
+    e = cudaLaunchKernelEx(&cfg, kern, std::forward<A>(args)...);
+  }
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    set_error("launch of %s failed: %s", name, cudaGetErrorString(e));
+    return QUIP_ERR_CUDA;
+  }
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  return QUIP_OK;
+}
+
+// ---- entry points shared between the .cu files --------------------------------
+// quip_config switches
+extern int g_gather_rows, g_pass_min_tiles, g_fewtok;                     // rot.cu
+extern int g_fewtok_max_m;                                                // rot_fewtok.cu: token count up to which the few-token kernels run
+extern int g_gv_rbc, g_gv_persist, g_gv_int, g_gv_tma, g_gv_cw, g_gv_stream;  // qgemv.cu
+
+// contractions (qgemm_skinny.cu, qgemv.cu, qgemm_tc.cu)
+int qgemm_skinny(const QuipLinearDesc* d, const __half* x, const __half* bias, __half* z, int M, int ksplit,
+                 float* part, int* counters, cudaStream_t s);
+int skinny_pick_ksplit(int N, int K, int rows_per_cta, int M);
+size_t skinny_workspace_bytes(int N, int M, int ksplit);
+int qgemv(const QuipLinearDesc* d, const __half* x, const __half* bias, __half* z, int M, cudaStream_t s);
+bool qgemv_fits(int K, int M, int bits);
+int qgemm_tc(const QuipLinearDesc* d, const __half* x, const float* xsum, const __half* bias, __half* z, int M,
+             cudaStream_t s);
+
+// passes and gathers (rot_fewtok.cu, rot_small.cu, rot_side.cu, rot_side_fewtok.cu, qgemm_tc.cu)
+bool pass_fewtok_ok(const QuipPass* ps, int64_t M, int n);
+int pass_fewtok(const QuipPass* ps, const __half* in, __half* out, int64_t M, int n, const int32_t* in_idx,
+                const float* in_scale, const int32_t* out_inv, const __half* out_bias, cudaStream_t s);
+int gather_fewtok(const __half* in, __half* out, int64_t M, int n, const int32_t* idx, const float* scale,
+                  const __half* bias, cudaStream_t s);
+int launch_small_fast(const QuipPass* ps, const __half* in, __half* out, int64_t M, int n, cudaStream_t s, bool* handled);
+int pass_big_tc(const QuipPass* ps, const __half* in, __half* out, int64_t M, int n, cudaStream_t s);
+bool side_fused_ok(const QuipSide* sd, int n);
+int side_fused(const QuipSide* sd, const __half* in, __half* out, int64_t M, const int32_t* in_idx, const float* in_scale,
+               const int32_t* out_idx, const __half* out_bias, float* xsum, cudaStream_t s);
+bool side_fewtok_ok(const QuipSide* sd, int n, int64_t M);   // both passes of a side in one launch, M <= 8
+int side_fewtok(const QuipSide* sd, const __half* in, __half* out, int64_t M, int n, const int32_t* in_idx,
+                const float* in_scale, const int32_t* out_inv, const __half* out_bias, cudaStream_t s);
 
 constexpr int SB_ROWS = 16;   // super-block: 16 rows x 128 k  (oracle/packing.py)
 constexpr int SB_K = 128;

@@ -215,11 +215,8 @@ extern "C" int quip_rmsnorm(const void* x, const void* residual, const void* wei
   const int nvec = d / 8;
   int threads = ((nvec + RN_MAXV - 1) / RN_MAXV + 31) / 32 * 32;
   QUIP_CHECK_ARG(threads <= 1024, "quip_rmsnorm: width %d exceeds %d", d, 1024 * RN_MAXV * 8);
-  rmsnorm_kernel<<<(unsigned)rows, threads, 0, (cudaStream_t)stream>>>((const __half*)x, (const __half*)residual,
-                                                                        (const __half*)weight, (__half*)sum_out,
-                                                                        (__half*)y, d, eps);
-  QUIP_LAUNCHED("rmsnorm_kernel");
-  return QUIP_OK;
+  return launch("rmsnorm_kernel", rmsnorm_kernel, (unsigned)rows, threads, 0, (cudaStream_t)stream, false, (const __half*)x,
+                (const __half*)residual, (const __half*)weight, (__half*)sum_out, (__half*)y, d, eps);
 }
 
 extern "C" int quip_rope(void* q, void* k, const void* cos, const void* sin, int64_t rows, int32_t n_q_heads,
@@ -230,11 +227,8 @@ extern "C" int quip_rope(void* q, void* k, const void* cos, const void* sin, int
   QUIP_CHECK_ARG(aligned16(q) && aligned16(k) && aligned16(cos) && aligned16(sin), "quip_rope: pointers must be 16-byte aligned");
   if (rows <= 0) return QUIP_OK;
   const int64_t items = rows * (n_q_heads + n_kv_heads) * (head_dim / 16);
-  rope_kernel<<<stream_grid(items, 256), 256, 0, (cudaStream_t)stream>>>((__half*)q, (__half*)k, (const __half*)cos,
-                                                                          (const __half*)sin, rows, n_q_heads,
-                                                                          n_kv_heads, head_dim);
-  QUIP_LAUNCHED("rope_kernel");
-  return QUIP_OK;
+  return launch("rope_kernel", rope_kernel, stream_grid(items, 256), 256, 0, (cudaStream_t)stream, false, (__half*)q,
+                (__half*)k, (const __half*)cos, (const __half*)sin, rows, n_q_heads, n_kv_heads, head_dim);
 }
 
 extern "C" int quip_silu_mul(const void* gate, const void* up, void* out, int64_t n, void* stream) {
@@ -242,10 +236,8 @@ extern "C" int quip_silu_mul(const void* gate, const void* up, void* out, int64_
   QUIP_CHECK_ARG(n >= 0 && n % 8 == 0, "quip_silu_mul: element count must be a multiple of 8");
   QUIP_CHECK_ARG(aligned16(gate) && aligned16(up) && aligned16(out), "quip_silu_mul: pointers must be 16-byte aligned");
   if (n == 0) return QUIP_OK;
-  silu_mul_kernel<<<stream_grid(n / 8, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)gate, (const __half*)up,
-                                                                             (__half*)out, n / 8);
-  QUIP_LAUNCHED("silu_mul_kernel");
-  return QUIP_OK;
+  return launch("silu_mul_kernel", silu_mul_kernel, stream_grid(n / 8, 256), 256, 0, (cudaStream_t)stream, false,
+                (const __half*)gate, (const __half*)up, (__half*)out, n / 8);
 }
 
 extern "C" int quip_silu_mul_gather(const void* gate, const void* up, const uint32_t* idx, void* out, int64_t rows, int32_t n,
@@ -258,15 +250,6 @@ extern "C" int quip_silu_mul_gather(const void* gate, const void* up, const uint
   const int rpc = (size_t)2 * SG_ROWS * n * sizeof(__half) <= 110 * 1024 ? SG_ROWS : 1;      // two CTAs per SM when they fit
   const size_t smem = (size_t)2 * rpc * n * sizeof(__half);
   QUIP_CHECK_ARG(smem <= 220 * 1024, "quip_silu_mul_gather: width %d does not fit shared memory", n);
-  static size_t done[64] = {0};
-  int dev = 0;
-  QUIP_CUDA(cudaGetDevice(&dev));
-  if (smem > 48 * 1024 && smem > done[dev & 63]) {
-    QUIP_CUDA(cudaFuncSetAttribute(silu_mul_gather_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    done[dev & 63] = smem;
-  }
-  silu_mul_gather_kernel<<<(unsigned)ceil_div(rows, rpc), SG_THREADS, smem, (cudaStream_t)stream>>>(
-      (const __half*)gate, (const __half*)up, idx, (__half*)out, rows, n, rpc);
-  QUIP_LAUNCHED("silu_mul_gather_kernel");
-  return QUIP_OK;
+  return launch("silu_mul_gather_kernel", silu_mul_gather_kernel, (unsigned)ceil_div(rows, rpc), SG_THREADS, smem,
+                (cudaStream_t)stream, false, (const __half*)gate, (const __half*)up, idx, (__half*)out, rows, n, rpc);
 }

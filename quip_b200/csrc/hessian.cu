@@ -148,14 +148,6 @@ extern "C" int quip_hessian_accumulate(const void* x, double* H, int64_t tokens,
   const int ntile = ceil_div(K, HS_TILE);
   const int64_t nct = (int64_t)ntile * (ntile + 1) / 2;
   const size_t smem = (size_t)2 * HS_STAGES * HS_TOK * HS_LD * sizeof(__half);
-  static bool done[64] = {false};
-  int dev = 0;
-  QUIP_CUDA(cudaGetDevice(&dev));
-  if (!done[dev & 63]) {
-    QUIP_CUDA(cudaFuncSetAttribute(hessian_syrk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    done[dev & 63] = true;
-  }
-  hessian_syrk_kernel<<<(unsigned)nct, HS_THREADS, smem, (cudaStream_t)stream>>>((const __half*)x, H, (int)tokens, K, ntile);
-  QUIP_LAUNCHED("hessian_syrk_kernel");
-  return QUIP_OK;
+  return launch("hessian_syrk_kernel", hessian_syrk_kernel, (unsigned)nct, HS_THREADS, smem, (cudaStream_t)stream, false,
+                (const __half*)x, H, (int)tokens, K, ntile);
 }

@@ -126,20 +126,6 @@ greedy_block_kernel(const float* __restrict__ preT, const float* __restrict__ Hb
 
 size_t lq_smem(int cnt) { return ((size_t)cnt * (cnt + 1) + (size_t)cnt * LQ_LD) * sizeof(float); }
 
-template <class K>
-int lq_prepare(K kern, int cnt) {
-  static size_t done[64] = {0};
-  int dev = 0;
-  QUIP_CUDA(cudaGetDevice(&dev));
-  dev &= 63;
-  const size_t smem = lq_smem(cnt);
-  if (smem > 48 * 1024 && smem > done[dev]) {
-    QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lq_smem(LQ_BLOCK)));
-    done[dev] = lq_smem(LQ_BLOCK);
-  }
-  return QUIP_OK;
-}
-
 }  // namespace
 
 }  // namespace quip
@@ -151,20 +137,14 @@ extern "C" int quip_ldlq_block(const float* baseT, const float* wT, const float*
   QUIP_CHECK_ARG(baseT && wT && Lb && qT && errT, "quip_ldlq_block: null pointer");
   QUIP_CHECK_ARG(cnt >= 1 && cnt <= LQ_BLOCK && m >= 1 && ld >= m && m < (1ll << 31), "quip_ldlq_block: bad sizes (cnt=%d)", cnt);
   QUIP_CHECK_ARG(bits >= 1 && bits <= 8, "quip_ldlq_block: bits out of range");
-  if (int e = lq_prepare(ldlq_block_kernel, cnt)) return e;
-  ldlq_block_kernel<<<(unsigned)ceil_div(m, LQ_ROWS), LQ_THREADS, lq_smem(cnt), (cudaStream_t)stream>>>(
-      baseT, wT, Lb, qT, errT, (int)m, (int)ld, cnt, (float)((1 << bits) - 1));
-  QUIP_LAUNCHED("ldlq_block_kernel");
-  return QUIP_OK;
+  return launch("ldlq_block_kernel", ldlq_block_kernel, (unsigned)ceil_div(m, LQ_ROWS), LQ_THREADS, lq_smem(cnt),
+                (cudaStream_t)stream, false, baseT, wT, Lb, qT, errT, (int)m, (int)ld, cnt, (float)((1 << bits) - 1));
 }
 
 extern "C" int quip_greedy_block(const float* preT, const float* Hb, float* wrT, float* sT, int64_t m, int64_t ld,
                                  int32_t cnt, void* stream) {
   QUIP_CHECK_ARG(preT && Hb && wrT && sT, "quip_greedy_block: null pointer");
   QUIP_CHECK_ARG(cnt >= 1 && cnt <= LQ_BLOCK && m >= 1 && ld >= m && m < (1ll << 31), "quip_greedy_block: bad sizes (cnt=%d)", cnt);
-  if (int e = lq_prepare(greedy_block_kernel, cnt)) return e;
-  greedy_block_kernel<<<(unsigned)ceil_div(m, LQ_ROWS), LQ_THREADS, lq_smem(cnt), (cudaStream_t)stream>>>(
-      preT, Hb, wrT, sT, (int)m, (int)ld, cnt);
-  QUIP_LAUNCHED("greedy_block_kernel");
-  return QUIP_OK;
+  return launch("greedy_block_kernel", greedy_block_kernel, (unsigned)ceil_div(m, LQ_ROWS), LQ_THREADS, lq_smem(cnt),
+                (cudaStream_t)stream, false, preT, Hb, wrT, sT, (int)m, (int)ld, cnt);
 }

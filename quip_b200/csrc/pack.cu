@@ -176,11 +176,8 @@ extern "C" int quip_pack_codes(const uint8_t* codes, int32_t N, int32_t K, int32
   int grid = ceil_div(total, 256);
   uint32_t* q = reinterpret_cast<uint32_t*>(qweight);
   if (bits == 3) QUIP_CUDA(cudaMemsetAsync(q, 0, quip_packed_words(N, K, 3) * 4, s));
-  if (bits == 2) pack_kernel<2><<<grid, 256, 0, s>>>(codes, N, K, q);
-  else if (bits == 3) pack_kernel<3><<<grid, 256, 0, s>>>(codes, N, K, q);
-  else pack_kernel<4><<<grid, 256, 0, s>>>(codes, N, K, q);
-  QUIP_LAUNCHED("pack_kernel");
-  return QUIP_OK;
+  auto kern = bits == 2 ? pack_kernel<2> : (bits == 3 ? pack_kernel<3> : pack_kernel<4>);
+  return launch("pack_kernel", kern, grid, 256, 0, s, false, codes, N, K, q);
 }
 
 extern "C" int quip_unpack_codes(const int32_t* qweight, int32_t N, int32_t K, int32_t bits, uint8_t* codes,
@@ -190,11 +187,8 @@ extern "C" int quip_unpack_codes(const int32_t* qweight, int32_t N, int32_t K, i
   cudaStream_t s = (cudaStream_t)stream;
   int grid = ceil_div((int64_t)N * K, 256);
   const uint32_t* q = reinterpret_cast<const uint32_t*>(qweight);
-  if (bits == 2) unpack_kernel<2><<<grid, 256, 0, s>>>(q, N, K, codes);
-  else if (bits == 3) unpack_kernel<3><<<grid, 256, 0, s>>>(q, N, K, codes);
-  else unpack_kernel<4><<<grid, 256, 0, s>>>(q, N, K, codes);
-  QUIP_LAUNCHED("unpack_kernel");
-  return QUIP_OK;
+  auto kern = bits == 2 ? unpack_kernel<2> : (bits == 3 ? unpack_kernel<3> : unpack_kernel<4>);
+  return launch("unpack_kernel", kern, grid, 256, 0, s, false, q, N, K, codes);
 }
 
 extern "C" int quip_convert_ref(const int32_t* ref_qweight, int32_t K, int32_t N, int32_t bits, uint8_t* codes,
@@ -205,9 +199,6 @@ extern "C" int quip_convert_ref(const int32_t* ref_qweight, int32_t K, int32_t N
   cudaStream_t s = (cudaStream_t)stream;
   int grid = ceil_div((int64_t)N * K, 256);
   const uint32_t* q = reinterpret_cast<const uint32_t*>(ref_qweight);
-  if (bits == 2) convert_ref_kernel<2><<<grid, 256, 0, s>>>(q, K, N, codes);
-  else if (bits == 3) convert_ref_kernel<3><<<grid, 256, 0, s>>>(q, K, N, codes);
-  else convert_ref_kernel<4><<<grid, 256, 0, s>>>(q, K, N, codes);
-  QUIP_LAUNCHED("convert_ref_kernel");
-  return QUIP_OK;
+  auto kern = bits == 2 ? convert_ref_kernel<2> : (bits == 3 ? convert_ref_kernel<3> : convert_ref_kernel<4>);
+  return launch("convert_ref_kernel", kern, grid, 256, 0, s, false, q, K, N, codes);
 }

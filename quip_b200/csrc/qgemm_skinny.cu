@@ -220,9 +220,6 @@ qgemm_skinny_kernel(const uint32_t* __restrict__ q, const __half* __restrict__ x
   }
 }
 
-int num_sms();
-static int sk_num_sms() { return num_sms(); }
-
 template <int BITS, int NT8, int RBC>
 static int launch_skinny(const QuipLinearDesc* d, const __half* x, const __half* bias, __half* z, int M,
                          int ksplit, float* part, int* counters, cudaStream_t s) {
@@ -232,22 +229,17 @@ static int launch_skinny(const QuipLinearDesc* d, const __half* x, const __half*
   constexpr int TOK = 8 * NT8, ROWS = 16 * RBC, RLD = ROWS + 8;
   size_t smem = (size_t)TOK * (per * 128 + SK_XPAD) * sizeof(__half) +
                 (size_t)(SK_WARPS * TOK * RLD + TOK) * sizeof(float);
-  auto kern = qgemm_skinny_kernel<BITS, NT8, RBC>;
   QUIP_CHECK_ARG(smem <= 220 * 1024, "skinny kernel: K slice too large (%zu B of shared memory)", smem);
-  QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   // persistent in the row dimension: ~2 CTAs per SM in total, each looping over row tiles with its K slice of
   // the activations staged once
   int tiles = ceil_div(d->N, ROWS);
   QUIP_CHECK_ARG(ksplit == 1 || tiles <= 4096, "skinny kernel: too many row tiles (%d) for split-K counters", tiles);
-  int gx = ceil_div(2 * sk_num_sms(), ksplit);
+  int gx = ceil_div(2 * num_sms(), ksplit);
   if (gx > tiles) gx = tiles;
   if (gx < 1) gx = 1;
-  dim3 grid(gx, ksplit);
-  kern<<<grid, SK_WARPS * 32, smem, s>>>(reinterpret_cast<const uint32_t*>(d->qweight), x, d->scales, d->zeros, bias,
-                                         z, M, d->K, d->N, per, (d->flags & QUIP_FLAG_SYMMETRIC) ? 1 : 0, part,
-                                         counters);
-  QUIP_LAUNCHED("qgemm_skinny_kernel");
-  return QUIP_OK;
+  return launch("qgemm_skinny_kernel", qgemm_skinny_kernel<BITS, NT8, RBC>, dim3(gx, ksplit), SK_WARPS * 32, smem, s, false,
+                reinterpret_cast<const uint32_t*>(d->qweight), x, d->scales, d->zeros, bias, z, M, d->K, d->N, per,
+                (d->flags & QUIP_FLAG_SYMMETRIC) ? 1 : 0, part, counters);
 }
 
 // Heuristic split.  Every K split costs a round trip of fp32 partials (write, fence, counter, the last CTA reads them all), and

@@ -249,18 +249,6 @@ static PFN_encodeTiled get_encode() {
   return fn;
 }
 
-static int g_num_sms = 0;
-
-int num_sms() {
-  if (!g_num_sms) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess ||
-        cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
-      g_num_sms = 148;
-  }
-  return g_num_sms;
-}
-
 // activations (rows, cols) fp16 row-major -> 2-D map, box {64 cols, box_rows}, 128B swizzle, zero OOB fill
 int make_act_map(CUtensorMap* tmap, const void* x, int64_t rows, int64_t cols, int box_rows) {
   PFN_encodeTiled enc = get_encode();
@@ -289,14 +277,10 @@ static int launch_tc(const QuipLinearDesc* d, const __half* x, const float* xsum
   using C = TcCfg<BN>;
   CUtensorMap tmap;
   if (int e = make_act_map(&tmap, x, M, d->K, BN)) return e;
-  auto kern = qgemm_tc_kernel<BITS, BN, false>;
-  QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-  int tiles = ceil_div(d->N, TC_BM) * ceil_div(M, BN);
-  int grid = tiles < num_sms() ? tiles : num_sms();
-  kern<<<grid, TC_THREADS, C::SMEM, s>>>(tmap, tmap, reinterpret_cast<const uint32_t*>(d->qweight), d->scales, d->zeros,
-                                         bias, xsum, z, M, d->K, d->N, (d->flags & QUIP_FLAG_SYMMETRIC) ? 1 : 0, 1, 0);
-  QUIP_LAUNCHED("qgemm_tc_kernel");
-  return QUIP_OK;
+  const int grid = std::min(ceil_div(d->N, TC_BM) * ceil_div(M, BN), num_sms());
+  return launch("qgemm_tc_kernel", qgemm_tc_kernel<BITS, BN, false>, grid, TC_THREADS, C::SMEM, s, false, tmap, tmap,
+                reinterpret_cast<const uint32_t*>(d->qweight), d->scales, d->zeros, bias, xsum, z, M, d->K, d->N,
+                (d->flags & QUIP_FLAG_SYMMETRIC) ? 1 : 0, 1, 0);
 }
 
 // block-diagonal pass with big contiguous blocks on the tensor cores (see DENSE in the kernel)
@@ -318,14 +302,9 @@ static int launch_tc_dense(const QuipPass* ps, const __half* in, __half* out, in
     set_error("cuTensorMapEncodeTiled (factors) failed with CUresult %d (p=%d nblk=%d)", (int)r, p, ps->nblk);
     return QUIP_ERR_CUDA;
   }
-  auto kern = qgemm_tc_kernel<2, BN, true>;
-  QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-  int tiles = ceil_div(p, BN) * ceil_div(M, TC_BM) * ps->nblk;
-  int grid = tiles < num_sms() ? tiles : num_sms();
-  kern<<<grid, TC_THREADS, C::SMEM, s>>>(tmx, tma, nullptr, nullptr, nullptr, nullptr, nullptr, out, M, p, p, 1,
-                                         ps->nblk, ps->shared ? 1 : 0);
-  QUIP_LAUNCHED("qgemm_tc_kernel<dense>");
-  return QUIP_OK;
+  const int grid = std::min(ceil_div(p, BN) * ceil_div(M, TC_BM) * ps->nblk, num_sms());
+  return launch("qgemm_tc_kernel<dense>", qgemm_tc_kernel<2, BN, true>, grid, TC_THREADS, C::SMEM, s, false, tmx, tma,
+                nullptr, nullptr, nullptr, nullptr, nullptr, out, M, p, p, 1, ps->nblk, ps->shared ? 1 : 0);
 }
 
 int pass_big_tc(const QuipPass* ps, const __half* in, __half* out, int64_t M, int n, cudaStream_t s) {

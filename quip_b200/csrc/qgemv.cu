@@ -891,39 +891,16 @@ qgemv_i8_tma_kernel(const uint32_t* __restrict__ q, const __half* __restrict__ x
   }
 }
 
-int num_sms();
-int launch_pdl(const void* kern, dim3 grid, dim3 block, size_t smem, cudaStream_t s, void** args);   // api.cu
-
 template <int BITS, int NT8, int RBC, int D>
 static int launch_gv(const QuipLinearDesc* d, const __half* x, const __half* bias, __half* z, int M, cudaStream_t s) {
   constexpr int TOK = 8 * NT8, ROWS = 16 * RBC, RLD = ROWS + 4;
   const size_t xs_bytes = ((size_t)M * (d->K + GV_XPAD) * sizeof(__half) + 15) & ~(size_t)15;
   const size_t smem = xs_bytes + (size_t)(2 * GV_WARPS * TOK * RLD + GV_WARPS * 2 * TOK) * sizeof(float);
   auto kern = qgemv_kernel<BITS, NT8, RBC, D>;
-  // the attribute and the occupancy query cost more host time than the kernel runs: cache per (kernel, device)
-  static size_t attr_smem[64] = {0}, occ_smem[64] = {0};
-  static int occ[64] = {0};
-  int dev = 0;
-  QUIP_CUDA(cudaGetDevice(&dev));
-  dev &= 63;
-  if (smem > attr_smem[dev]) {
-    QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_smem[dev] = smem;
-  }
-  const int tiles = ceil_div(d->N / 16, RBC);
-  int grid = tiles;
-  if (g_gv_persist) {
-    if (occ[dev] == 0 || occ_smem[dev] != smem) {
-      QUIP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ[dev], kern, GV_WARPS * 32, smem));
-      if (occ[dev] < 1) occ[dev] = 1;
-      occ_smem[dev] = smem;
-    }
-    if (grid > occ[dev] * num_sms()) grid = occ[dev] * num_sms();
-  }
-  kern<<<grid, GV_WARPS * 32, smem, s>>>(reinterpret_cast<const uint32_t*>(d->qweight), x, d->scales, d->zeros, bias,
-                                         z, M, d->K, d->N);
-  QUIP_LAUNCHED("qgemv_kernel");
-  return QUIP_OK;
+  int grid = ceil_div(d->N / 16, RBC);
+  if (g_gv_persist) grid = std::min(grid, blocks_per_sm((const void*)kern, GV_WARPS * 32, smem) * num_sms());
+  return launch("qgemv_kernel", kern, grid, GV_WARPS * 32, smem, s, false, reinterpret_cast<const uint32_t*>(d->qweight),
+                x, d->scales, d->zeros, bias, z, M, d->K, d->N);
 }
 
 template <int BITS, int NT8, int RBC, int D>
@@ -932,29 +909,10 @@ static int launch_gv_i8(const QuipLinearDesc* d, const __half* x, const __half* 
   const size_t limb_bytes = ((size_t)GV_LIMBS * M * (d->K + 32) + 15) & ~(size_t)15;
   const size_t smem = limb_bytes + (size_t)(2 * GV_WARPS * COLS * RLD) * sizeof(int) + (size_t)(16 + 2 * GV_WARPS) * sizeof(float);
   auto kern = qgemv_i8_kernel<BITS, NT8, RBC, D>;
-  static size_t attr_smem[64] = {0}, occ_smem[64] = {0};
-  static int occ[64] = {0};
-  int dev = 0;
-  QUIP_CUDA(cudaGetDevice(&dev));
-  dev &= 63;
-  if (smem > attr_smem[dev]) {
-    QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_smem[dev] = smem;
-  }
-  const int tiles = ceil_div(d->N / 16, RBC);
-  int grid = tiles;
-  if (g_gv_persist) {
-    if (occ[dev] == 0 || occ_smem[dev] != smem) {
-      QUIP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ[dev], kern, GV_WARPS * 32, smem));
-      if (occ[dev] < 1) occ[dev] = 1;
-      occ_smem[dev] = smem;
-    }
-    if (grid > occ[dev] * num_sms()) grid = occ[dev] * num_sms();
-  }
-  kern<<<grid, GV_WARPS * 32, smem, s>>>(reinterpret_cast<const uint32_t*>(d->qweight), x, d->scales, d->zeros, bias,
-                                         z, M, d->K, d->N);
-  QUIP_LAUNCHED("qgemv_i8_kernel");
-  return QUIP_OK;
+  int grid = ceil_div(d->N / 16, RBC);
+  if (g_gv_persist) grid = std::min(grid, blocks_per_sm((const void*)kern, GV_WARPS * 32, smem) * num_sms());
+  return launch("qgemv_i8_kernel", kern, grid, GV_WARPS * 32, smem, s, false,
+                reinterpret_cast<const uint32_t*>(d->qweight), x, d->scales, d->zeros, bias, z, M, d->K, d->N);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1078,30 +1036,9 @@ static int launch_gv_i8_stream(const QuipLinearDesc* d, const __half* x, const _
   const size_t limb_bytes = ((size_t)GV_LIMBS * M * (d->K + 32) + 15) & ~(size_t)15;
   const size_t smem = limb_bytes + (size_t)(16 + 10 * GS_WARPS) * sizeof(float);
   auto kern = qgemv_i8_stream_kernel<BITS, NT8>;
-  static size_t attr_smem[64] = {0};
-  static int occ[64] = {0};
-  int dev = 0;
-  QUIP_CUDA(cudaGetDevice(&dev));
-  dev &= 63;
-  if (smem > attr_smem[dev]) {
-    QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_smem[dev] = smem;
-    occ[dev] = 0;
-  }
-  if (occ[dev] == 0) {
-    QUIP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ[dev], kern, GS_WARPS * 32, smem));
-    if (occ[dev] < 1) occ[dev] = 1;
-  }
-  int grid = occ[dev] * num_sms();
-  const int need = ceil_div(d->N / 16, GS_WARPS);
-  if (grid > need) grid = need;
-  const uint32_t* qw = reinterpret_cast<const uint32_t*>(d->qweight);
-  const float *sc = d->scales, *ze = d->zeros;
-  int K = d->K, N = d->N;
-  void* args[] = {(void*)&qw, (void*)&x, (void*)&sc, (void*)&ze, (void*)&bias, (void*)&z, (void*)&M, (void*)&K, (void*)&N};
-  if (int e = launch_pdl((const void*)kern, dim3(grid), dim3(GS_WARPS * 32), smem, s, args)) return e;
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  return QUIP_OK;
+  const int grid = std::min(blocks_per_sm((const void*)kern, GS_WARPS * 32, smem) * num_sms(), ceil_div(d->N / 16, GS_WARPS));
+  return launch("qgemv_i8_stream_kernel", kern, grid, GS_WARPS * 32, smem, s, true,
+                reinterpret_cast<const uint32_t*>(d->qweight), x, d->scales, d->zeros, bias, z, M, d->K, d->N);
 }
 
 static bool gv_stream_fits(int K, int M) {
@@ -1120,24 +1057,9 @@ static int launch_gv_i8_tma(const QuipLinearDesc* d, const __half* x, const __ha
   if (ns > 12) ns = 12;
   QUIP_CHECK_ARG(ns >= 2 * RBC, "qgemv: K=%d with %d tokens leaves no room for the weight ring", d->K, M);
   const size_t smem = (size_t)ns * STAGE_BYTES + fixed + (size_t)(2 * ns + 4) * sizeof(uint64_t);
-  auto kern = qgemv_i8_tma_kernel<BITS, NT8, RBC, CW>;
-  static size_t attr_smem[64] = {0};
-  int dev = 0;
-  QUIP_CUDA(cudaGetDevice(&dev));
-  dev &= 63;
-  if (smem > attr_smem[dev]) {
-    QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_smem[dev] = smem;
-  }
-  const int tiles = ceil_div(d->N / 16, RBC);
-  const int grid = tiles < num_sms() ? tiles : num_sms();
-  const uint32_t* qw = reinterpret_cast<const uint32_t*>(d->qweight);
-  const float *sc = d->scales, *ze = d->zeros;
-  int K = d->K, N = d->N;
-  void* args[] = {(void*)&qw, (void*)&x, (void*)&sc, (void*)&ze, (void*)&bias, (void*)&z, (void*)&M, (void*)&K, (void*)&N, (void*)&ns};
-  if (int e = launch_pdl((const void*)kern, dim3(grid), dim3(gt_threads(CW)), smem, s, args)) return e;
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  return QUIP_OK;
+  const int grid = std::min(ceil_div(d->N / 16, RBC), num_sms());
+  return launch("qgemv_i8_tma_kernel", qgemv_i8_tma_kernel<BITS, NT8, RBC, CW>, grid, gt_threads(CW), smem, s, true,
+                reinterpret_cast<const uint32_t*>(d->qweight), x, d->scales, d->zeros, bias, z, M, d->K, d->N, ns);
 }
 
 // does the bulk-copy kernel have room for at least a minimal ring next to the token bytes?

@@ -389,23 +389,8 @@ using namespace quip;
 template <int R>
 static int launch_gather(const __half* in, __half* out, int64_t M, int n, const int32_t* idx, const float* scale,
                          const __half* bias, cudaStream_t s) {
-  size_t smem = (size_t)R * n * sizeof(__half);
-  auto kern = gather_kernel<R>;
-  if (smem > 48 * 1024) QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<ceil_div(M, R), 256, smem, s>>>(in, out, M, n, idx, scale, bias);
-  QUIP_LAUNCHED("gather_kernel");
-  return QUIP_OK;
-}
-
-namespace quip {
-extern int g_fewtok_max_m;
-bool pass_fewtok_ok(const QuipPass* ps, int64_t M, int n);
-int pass_fewtok(const QuipPass* ps, const __half* in, __half* out, int64_t M, int n, const int32_t* in_idx,
-                const float* in_scale, const int32_t* out_inv, const __half* out_bias, cudaStream_t s);
-int gather_fewtok(const __half* in, __half* out, int64_t M, int n, const int32_t* idx, const float* scale,
-                  const __half* bias, cudaStream_t s);
-int pass_big_tc(const QuipPass* ps, const __half* in, __half* out, int64_t M, int n, cudaStream_t s);
-int launch_small_fast(const QuipPass* ps, const __half* in, __half* out, int64_t M, int n, cudaStream_t s, bool* handled);
+  return launch("gather_kernel", gather_kernel<R>, ceil_div(M, R), 256, (size_t)R * n * sizeof(__half), s, false, in, out,
+                M, n, idx, scale, bias);
 }
 
 extern "C" int quip_gather(const void* in, void* out, int64_t M, int32_t n, const int32_t* idx,
@@ -431,9 +416,8 @@ extern "C" int quip_gather(const void* in, void* out, int64_t M, int32_t n, cons
 
 extern "C" int quip_rowsum(const void* x, float* xsum, int64_t M, int32_t K, void* stream) {
   QUIP_CHECK_ARG(x && xsum && M > 0 && K > 0 && K % 8 == 0, "rowsum: bad arguments");
-  rowsum_kernel<<<ceil_div(M, 8), 256, 0, (cudaStream_t)stream>>>((const __half*)x, xsum, M, K);
-  QUIP_LAUNCHED("rowsum_kernel");
-  return QUIP_OK;
+  return launch("rowsum_kernel", rowsum_kernel, ceil_div(M, 8), 256, 0, (cudaStream_t)stream, false, (const __half*)x, xsum,
+                M, K);
 }
 
 template <int P>
@@ -445,10 +429,8 @@ static int launch_small(const QuipPass* ps, const __half* in, __half* out, int64
   while (tok_chunk > 16 && (int64_t)groups * ceil_div(M, tok_chunk) < 296) tok_chunk >>= 1;
   int vec = ps->strided ? (ps->nblk % 8 == 0) : (ps->p % 8 == 0 && n % 8 == 0);
   dim3 grid(groups, ceil_div(M, tok_chunk));
-  pass_small_kernel<P><<<grid, 256, 0, s>>>(in, out, (const __half*)ps->factors, M, n, ps->p, ps->nblk,
-                                             ps->strided, ps->shared, tok_chunk, vec);
-  QUIP_LAUNCHED("pass_small_kernel");
-  return QUIP_OK;
+  return launch("pass_small_kernel", pass_small_kernel<P>, grid, 256, 0, s, false, in, out, (const __half*)ps->factors, M, n,
+                ps->p, ps->nblk, ps->strided, ps->shared, tok_chunk, vec);
 }
 
 extern "C" int quip_rot_pass(const QuipPass* ps, const void* in_, void* out_, int64_t M, int32_t n, int impl,
@@ -477,12 +459,10 @@ extern "C" int quip_rot_pass(const QuipPass* ps, const void* in_, void* out_, in
   if (impl != 1 && impl != 3 && big_ok && M > 32 && ((((uintptr_t)in | (uintptr_t)out | (uintptr_t)ps->factors) & 15) == 0))
     return pass_big_tc(ps, in, out, M, n, s);      // tcgen05: the 688x688 blocks of an 11008 side are real GEMMs
   if (impl != 1 && big_ok) {
-    size_t smem = (size_t)BIG_STAGES * (BIG_BM + BIG_BN) * BIG_LD * sizeof(__half);
-    QUIP_CUDA(cudaFuncSetAttribute(pass_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dim3 grid(ceil_div(p, BIG_BN), ceil_div(M, BIG_BM), ps->nblk);
-    pass_big_kernel<<<grid, 256, smem, s>>>(in, out, (const __half*)ps->factors, M, n, p, ps->shared);
-    QUIP_LAUNCHED("pass_big_kernel");
-    return QUIP_OK;
+    const size_t smem = (size_t)BIG_STAGES * (BIG_BM + BIG_BN) * BIG_LD * sizeof(__half);
+    const dim3 grid(ceil_div(p, BIG_BN), ceil_div(M, BIG_BM), ps->nblk);
+    return launch("pass_big_kernel", pass_big_kernel, grid, 256, smem, s, false, in, out, (const __half*)ps->factors, M, n, p,
+                  ps->shared);
   }
   if (impl == 2) {
     set_error("rot_pass: no tensor-core kernel for p=%d strided=%d", p, ps->strided);
@@ -490,10 +470,6 @@ extern "C" int quip_rot_pass(const QuipPass* ps, const void* in_, void* out_, in
   }
   size_t smem = (size_t)n * sizeof(float);
   QUIP_CHECK_ARG(smem <= 200 * 1024, "rot_pass: n=%d too large for the generic kernel", n);
-  if (smem > 48 * 1024)
-    QUIP_CUDA(cudaFuncSetAttribute(pass_simple_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  pass_simple_kernel<<<(unsigned)M, 256, smem, s>>>(in, out, (const __half*)ps->factors, n, p, ps->nblk, ps->strided,
-                                                    ps->shared);
-  QUIP_LAUNCHED("pass_simple_kernel");
-  return QUIP_OK;
+  return launch("pass_simple_kernel", pass_simple_kernel, (unsigned)M, 256, smem, s, false, in, out, (const __half*)ps->factors,
+                n, p, ps->nblk, ps->strided, ps->shared);
 }

@@ -229,8 +229,6 @@ gather_fewtok_kernel(const __half* __restrict__ in, __half* __restrict__ out, in
   }
 }
 
-int launch_pdl(const void* kern, dim3 grid, dim3 block, size_t smem, cudaStream_t s, void** args);   // api.cu
-
 int g_fewtok_max_m = 32;      // 9..32 tokens (batched decode) through the few-token kernels too; quip_config("fewtok_max_m", 8)
                               // sends them to the many-token route instead
 
@@ -253,40 +251,17 @@ int pass_fewtok(const QuipPass* ps, const __half* in, __half* out, int64_t M, in
   if (nb_cta > ps->nblk) nb_cta = ps->nblk;
   QUIP_CHECK_ARG(nb_cta * p <= FT_XPT * FT_WARPS * 32, "few-token pass: %d blocks of %d per CTA exceed the staging budget", nb_cta, p);
   const size_t smem = (size_t)M * (nb_cta * p + 16) * sizeof(__half);
-  const int Mi = (int)M, nblk = ps->nblk, strided = ps->strided, shared = ps->shared;
-  const __half* F = (const __half*)ps->factors;
-  void* args[] = {(void*)&in, (void*)&out, (void*)&F, (void*)&Mi, (void*)&n, (void*)&p, (void*)&nblk,
-                  (void*)&strided, (void*)&shared, (void*)&kparts, (void*)&steps_per_part, (void*)&in_idx,
-                  (void*)&in_scale, (void*)&out_inv, (void*)&out_bias, (void*)&nb_cta};
-  const void* kern = M <= 8 ? (const void*)pass_fewtok_kernel<1>
-                            : (M <= 16 ? (const void*)pass_fewtok_kernel<2> : (const void*)pass_fewtok_kernel<4>);
-  // the kernel also holds NG x FT_WARPS x 16 x 9 floats of static shared memory (the k-part reduction): the 48 KiB default
-  // limit applies to the sum
-  const size_t smem_static = (size_t)(M <= 8 ? 1 : (M <= 16 ? 2 : 4)) * FT_WARPS * 16 * 9 * sizeof(float);
-  if (smem + smem_static > 48 * 1024) {                    // many tokens x two 688-wide blocks: opt in once per device
-    QUIP_CHECK_ARG(smem <= 200 * 1024, "few-token pass: %zu bytes of token staging", smem);
-    static bool attr_done[64][3] = {};
-    int dev = 0;
-    QUIP_CUDA(cudaGetDevice(&dev));
-    const int ki = M <= 8 ? 0 : (M <= 16 ? 1 : 2);
-    if (!attr_done[dev & 63][ki]) {
-      QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      attr_done[dev & 63][ki] = true;
-    }
-  }
-  if (int e = launch_pdl(kern, dim3((unsigned)ceil_div(groups, per_cta)), dim3(FT_WARPS * 32), smem, s, args))
-    return e;
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  return QUIP_OK;
+  QUIP_CHECK_ARG(smem <= 200 * 1024, "few-token pass: %zu bytes of token staging", smem);
+  auto kern = M <= 8 ? pass_fewtok_kernel<1> : (M <= 16 ? pass_fewtok_kernel<2> : pass_fewtok_kernel<4>);
+  return launch("pass_fewtok_kernel", kern, (unsigned)ceil_div(groups, per_cta), FT_WARPS * 32, smem, s, true, in, out,
+                (const __half*)ps->factors, (int)M, n, p, ps->nblk, ps->strided, ps->shared, kparts, steps_per_part, in_idx,
+                in_scale, out_inv, out_bias, nb_cta);
 }
 
 int gather_fewtok(const __half* in, __half* out, int64_t M, int n, const int32_t* idx, const float* scale,
                   const __half* bias, cudaStream_t s) {
-  const int Mi = (int)M;
-  void* args[] = {(void*)&in, (void*)&out, (void*)&Mi, (void*)&n, (void*)&idx, (void*)&scale, (void*)&bias};
-  if (int e = launch_pdl((const void*)gather_fewtok_kernel, dim3((unsigned)ceil_div(n / 8, 128)), dim3(128), 0, s, args)) return e;
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  return QUIP_OK;
+  return launch("gather_fewtok_kernel", gather_fewtok_kernel, (unsigned)ceil_div(n / 8, 128), 128, 0, s, true, in, out,
+                (int)M, n, idx, scale, bias);
 }
 
 }  // namespace quip

@@ -404,21 +404,9 @@ template <int PA, int PB>
 static int launch_side(const __half* in, __half* out, int64_t M, const int32_t* in_idx, const float* in_scale,
                        const int32_t* out_idx, const __half* out_bias, const QuipPass* col, const QuipPass* row,
                        int col_first, float* xsum, cudaStream_t s) {
-  using C = SideCfg<PA, PB>;
-  auto kern = side_fused_kernel<PA, PB>;
-  static bool attr_done[64] = {false};
-  int dev = 0;
-  QUIP_CUDA(cudaGetDevice(&dev));
-  dev &= 63;
-  if (!attr_done[dev]) {
-    QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    attr_done[dev] = true;
-  }
-  kern<<<(unsigned)ceil_div(M, SD_TOK), SD_WARPS * 32, C::SMEM, s>>>(
-      in, out, M, in_idx, in_scale, out_idx, out_bias, (const uint4*)col->factors_frag, col->shared,
-      (const uint4*)row->factors_frag, row->shared, col_first, xsum);
-  QUIP_LAUNCHED("side_fused_kernel");
-  return QUIP_OK;
+  return launch("side_fused_kernel", side_fused_kernel<PA, PB>, (unsigned)ceil_div(M, SD_TOK), SD_WARPS * 32,
+                SideCfg<PA, PB>::SMEM, s, false, in, out, M, in_idx, in_scale, out_idx, out_bias,
+                (const uint4*)col->factors_frag, col->shared, (const uint4*)row->factors_frag, row->shared, col_first, xsum);
 }
 
 // Can this side (two passes) run as one fused kernel?  One strided pass of p = PA over PB blocks and one contiguous

@@ -270,8 +270,6 @@ side_fewtok_kernel(const __half* __restrict__ in, __half* __restrict__ out, int 
 
 }  // namespace
 
-int launch_pdl(const void* kern, dim3 grid, dim3 block, size_t smem, cudaStream_t s, void** args);   // api.cu
-
 constexpr size_t SF_SMEM_MAX = 224 * 1024;
 static int sf_blocks_per_cta(int p1) { return p1 <= 16 ? 4 : 1; }
 static int sf_rows_per_cta(int p1) { return p1 <= 64 ? p1 : (p1 > 512 ? SF_ROWS : 64); }
@@ -307,31 +305,12 @@ int side_fewtok(const QuipSide* sd, const __half* in, __half* out, int64_t M, in
   const int rtiles = ceil_div(b.p, rows_per_cta);
   const int items = ceil_div(b.nblk, blocks_per_cta) * rtiles;
   const size_t smem = side_fewtok_smem(n, a, b, (int)M);
-  const void* kern = nullptr;
-  switch ((int)M) {
-    case 1: kern = (const void*)side_fewtok_kernel<1>; break;
-    case 2: kern = (const void*)side_fewtok_kernel<2>; break;
-    case 3: kern = (const void*)side_fewtok_kernel<3>; break;
-    case 4: kern = (const void*)side_fewtok_kernel<4>; break;
-    case 5: kern = (const void*)side_fewtok_kernel<5>; break;
-    case 6: kern = (const void*)side_fewtok_kernel<6>; break;
-    case 7: kern = (const void*)side_fewtok_kernel<7>; break;
-    default: kern = (const void*)side_fewtok_kernel<8>; break;
-  }
-  if (smem > 48 * 1024) {
-    static bool done[64][SF_MAXTOK + 1] = {};
-    int dev = 0;
-    QUIP_CUDA(cudaGetDevice(&dev));
-    if (!done[dev & 63][M]) {
-      QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_SMEM_MAX));
-      done[dev & 63][M] = true;
-    }
-  }
-  void* args[] = {(void*)&in, (void*)&out, (void*)&n, (void*)&P0, (void*)&P1, (void*)&in_idx, (void*)&in_scale,
-                  (void*)&out_inv, (void*)&out_bias, (void*)&rows_per_cta, (void*)&blocks_per_cta};
-  if (int e = launch_pdl(kern, dim3((unsigned)items), dim3(SF_THREADS), smem, s, args)) return e;
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  return QUIP_OK;
+  QUIP_CHECK_ARG(M >= 1 && M <= SF_MAXTOK, "few-token side: %lld tokens", (long long)M);
+  static constexpr decltype(&side_fewtok_kernel<1>) kerns[SF_MAXTOK] = {
+      side_fewtok_kernel<1>, side_fewtok_kernel<2>, side_fewtok_kernel<3>, side_fewtok_kernel<4>,
+      side_fewtok_kernel<5>, side_fewtok_kernel<6>, side_fewtok_kernel<7>, side_fewtok_kernel<8>};
+  return launch("side_fewtok_kernel", kerns[M - 1], (unsigned)items, SF_THREADS, smem, s, true, in, out, n, P0, P1, in_idx,
+                in_scale, out_inv, out_bias, rows_per_cta, blocks_per_cta);
 }
 
 }  // namespace quip

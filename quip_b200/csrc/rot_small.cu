@@ -303,7 +303,6 @@ pass_strided_kernel(const __half* __restrict__ in, __half* __restrict__ out, con
 }
 
 // ------------------------------------------------------------------------------------------------
-extern int g_pass_min_tiles;
 static int pick_tok_chunk(int64_t M, int gx, int tm) {
   // enough CTAs for ~2 per SM, but keep >= 4 tiles per CTA when M allows so the register-resident
   // factors are amortised
@@ -324,10 +323,8 @@ static int launch_fast(const QuipPass* ps, const __half* in, __half* out, int64_
     size_t smem = (size_t)PC_WARPS * PC_STAGES * C::BPW * C::TM * C::LD * sizeof(__half);
     const bool affine = (32 % (C::BPW * ps->p / 8)) == 0;
     auto kern = affine ? pass_contig_kernel<P, true> : pass_contig_kernel<P, false>;
-    if (smem > 48 * 1024) QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dim3 grid(gx, ceil_div(M, tok_chunk));
-    kern<<<grid, PC_WARPS * 32, smem, s>>>(in, out, F, M, n, ps->p, ps->nblk, ps->shared, tok_chunk);
-    QUIP_LAUNCHED("pass_contig_kernel");
+    return launch("pass_contig_kernel", kern, dim3(gx, ceil_div(M, tok_chunk)), PC_WARPS * 32, smem, s, false, in, out, F, M,
+                  n, ps->p, ps->nblk, ps->shared, tok_chunk);
   } else {
     // 64-wide blocks: 16 warps = 16 adjacent blocks per CTA, so the strided runs are full 32-byte sectors
     constexpr int W = (P == 64) ? 16 : 8;
@@ -337,12 +334,9 @@ static int launch_fast(const QuipPass* ps, const __half* in, __half* out, int64_
     size_t smem = (size_t)2 * GB * PS_TM * C::LD * sizeof(__half);
     const bool affine = ((W * 32) % ((ps->p / 2) * (GB / 8))) == 0;
     auto kern = affine ? pass_strided_kernel<P, true, W> : pass_strided_kernel<P, false, W>;
-    if (smem > 48 * 1024) QUIP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dim3 grid(gx, ceil_div(M, tok_chunk));
-    kern<<<grid, W * 32, smem, s>>>(in, out, F, M, n, ps->p, ps->nblk, ps->shared, tok_chunk);
-    QUIP_LAUNCHED("pass_strided_kernel");
+    return launch("pass_strided_kernel", kern, dim3(gx, ceil_div(M, tok_chunk)), W * 32, smem, s, false, in, out, F, M, n,
+                  ps->p, ps->nblk, ps->shared, tok_chunk);
   }
-  return QUIP_OK;
 }
 
 // Fast path for p <= 64 when the 16-byte vector conditions hold; otherwise *handled stays false and the

@@ -96,8 +96,6 @@ vecquant_kernel(const float* __restrict__ vec, const uint32_t* __restrict__ mat,
 
 }  // namespace
 
-int num_sms();
-
 }  // namespace quip
 
 using namespace quip;
@@ -119,9 +117,6 @@ extern "C" int quip_vecquant_matmul(const float* vec, const int32_t* mat, float*
   dim3 grid((unsigned)col_ctas, (unsigned)ksplit);
   cudaStream_t s = (cudaStream_t)stream;
   const uint32_t* m = reinterpret_cast<const uint32_t*>(mat);
-  if (bits == 3) vecquant_kernel<3><<<grid, VQ_THREADS, smem, s>>>(vec, m, mul, scales, zeros, K, N, per);
-  else if (bits == 4) vecquant_kernel<4><<<grid, VQ_THREADS, smem, s>>>(vec, m, mul, scales, zeros, K, N, per);
-  else vecquant_kernel<2><<<grid, VQ_THREADS, smem, s>>>(vec, m, mul, scales, zeros, K, N, per);
-  QUIP_LAUNCHED("vecquant_kernel");
-  return QUIP_OK;
+  auto kern = bits == 3 ? vecquant_kernel<3> : (bits == 4 ? vecquant_kernel<4> : vecquant_kernel<2>);
+  return launch("vecquant_kernel", kern, grid, VQ_THREADS, smem, s, false, vec, m, mul, scales, zeros, K, N, per);
 }
