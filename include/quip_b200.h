@@ -135,6 +135,22 @@ int quip_silu_mul(const void* gate, const void* up, void* out, int64_t n, void* 
 int quip_silu_mul_gather(const void* gate, const void* up, const uint32_t* idx, void* out, int64_t rows, int32_t n,
                          void* stream);
 
+/* One decode step of attention for `batch` sequences over a static KV cache (quip_b200/generate.py).  fp16 tensors,
+ * 16-byte aligned: q (batch, n_heads*head_dim) and k_new, v_new (batch, n_kv_heads*head_dim) token-major, as the
+ * projections produce them (after rotary for Llama; q already scaled for OPT); k_cache, v_cache (batch, n_kv_heads,
+ * max_len, head_dim); pos (batch) int32, the position this step writes.  Sequence b stores k_new / v_new at pos[b] and
+ * attends to positions 0 .. pos[b]:  out (batch, n_heads*head_dim) = softmax(scale * q K^T) V, softmax and sums in fp32,
+ * the query heads h of a KV head being h / (n_heads / n_kv_heads).  Only valid cache rows are read; long contexts are
+ * split along the sequence and the fp32 partials, kept in the workspace, are merged in a fixed order (deterministic).
+ * head_dim 64 or 128 and 1, 2, 4 or 8 query heads per KV head, else QUIP_ERR_UNSUPPORTED.  pos[b] must lie in
+ * 0 .. max_len-1 (the caller's check); a row outside it is not stored and its output is NaN. */
+int quip_decode_attention(const void* q, const void* k_new, const void* v_new, void* k_cache, void* v_cache,
+                          const int32_t* pos, int32_t batch, int32_t n_heads, int32_t n_kv_heads, int32_t max_len,
+                          int32_t head_dim, float scale, void* out, void* workspace, size_t workspace_bytes,
+                          void* stream);
+int quip_decode_attention_workspace_bytes(int32_t batch, int32_t n_heads, int32_t max_len, int32_t head_dim,
+                                          size_t* out_bytes);
+
 /* Signature-compatible replacement of the reference's own native call (quant_cuda.vecquant3matmul quant.py:229-230,
  * vecquant4matmul zeroShot/models/quant.py:207-208): ONE token, fp32, on the REFERENCE's packed layout
  * (bits 3: int32 (K*3/32, N) as Quant3Linear.pack writes it; bits 4: (K/8, N); bits 2: (K/16, N)):

@@ -56,6 +56,10 @@ EXPORTS = {
     'quip_greedy_block': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_void_p]),
     'quip_hessian_accumulate': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
     'quip_silu_mul_gather': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
+    'quip_decode_attention': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                        C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_void_p, C.c_void_p,
+                                        C.c_size_t, C.c_void_p]),
+    'quip_decode_attention_workspace_bytes': (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_size_t)]),
     'quip_pack_codes': (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     'quip_unpack_codes': (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     'quip_convert_ref': (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),

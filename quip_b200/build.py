@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 OBJ = os.path.join(HERE, 'build')
 LIB = os.path.join(HERE, 'libquip_b200.so')
-SOURCES = ['api.cu', 'pack.cu', 'rot.cu', 'rot_small.cu', 'rot_fewtok.cu', 'rot_side.cu', 'rot_side_fewtok.cu', 'glue.cu', 'vecquant.cu', 'ldlq.cu', 'hessian.cu', 'qgemm_skinny.cu', 'qgemv.cu', 'qgemm_tc.cu']
+SOURCES = ['api.cu', 'pack.cu', 'rot.cu', 'rot_small.cu', 'rot_fewtok.cu', 'rot_side.cu', 'rot_side_fewtok.cu', 'glue.cu', 'vecquant.cu', 'ldlq.cu', 'hessian.cu', 'qgemm_skinny.cu', 'qgemv.cu', 'qgemm_tc.cu', 'attn_decode.cu']
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
 FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
          '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr']

@@ -103,6 +103,27 @@ class GraphDecoder:
         self.k_cache.zero_()
         self.v_cache.zero_()
 
+    # ---- attention of the step, shared by the three kinds of glue (quip_b200.generate.Generator overrides both)
+    def _attn_context(self):
+        """What _attend needs of the step's positions, computed once per step: the mask over the static cache."""
+        return (self._arange <= self.position)[None, None, None, :]                     # (1, 1, 1, max_len)
+
+    def _attend(self, li, q, k, v, scale, mask):
+        """q (B, nh, 1, hd), k, v (B, nkv, 1, hd) of the step: store k, v at the position in layer li's cache and attend over
+        the whole cache under the mask.  Returns (B, nh, 1, hd)."""
+        pos = self.position
+        self.k_cache[li].index_copy_(2, pos, k)
+        self.v_cache[li].index_copy_(2, pos, v)
+        kk, vv = self.k_cache[li], self.v_cache[li]
+        if self.nkv != self.nh:
+            kk = kk.repeat_interleave(self.nh // self.nkv, dim=1)
+            vv = vv.repeat_interleave(self.nh // self.nkv, dim=1)
+        return F.scaled_dot_product_attention(q, kk, vv, attn_mask=mask, scale=scale)
+
+    def _graph_generators(self):
+        """Random generators the step draws from, registered with the graph so that each replay advances them."""
+        return ()
+
     # ---- the layers of the stage, three kinds of glue.  Each takes the hidden state entering the stage and returns
     # (h, pend): the residual stream and a branch output still to be added to it (None when already added).
 
@@ -115,7 +136,7 @@ class GraphDecoder:
         h = h.contiguous()
         cos = self.cos.index_select(0, pos).expand(B, hd).contiguous()                     # one row per sequence
         sin = self.sin.index_select(0, pos).expand(B, hd).contiguous()
-        mask = (self._arange <= pos)[None, None, None, :]
+        ctx = self._attn_context()
         pend = None
         for li, layer in enumerate(self.layers):
             a, mlp = layer.self_attn, layer.mlp
@@ -126,14 +147,8 @@ class GraphDecoder:
                 h, x = ops.rmsnorm(h, n1.weight, n1.variance_epsilon, residual=pend)
             q, k, v = self._parallel(x, [a.q_proj, a.k_proj, a.v_proj])
             ops.rope_(q, k, cos, sin, hd)
-            self.k_cache[li].index_copy_(2, pos, k.view(B, 1, nkv, hd).transpose(1, 2))
-            self.v_cache[li].index_copy_(2, pos, v.view(B, 1, nkv, hd).transpose(1, 2))
-            kk, vv = self.k_cache[li], self.v_cache[li]
-            if nkv != nh:
-                kk = kk.repeat_interleave(nh // nkv, dim=1)
-                vv = vv.repeat_interleave(nh // nkv, dim=1)
-            o = F.scaled_dot_product_attention(q.view(B, 1, nh, hd).transpose(1, 2), kk, vv, attn_mask=mask,
-                                               scale=1.0 / math.sqrt(hd))
+            o = self._attend(li, q.view(B, 1, nh, hd).transpose(1, 2), k.view(B, 1, nkv, hd).transpose(1, 2),
+                             v.view(B, 1, nkv, hd).transpose(1, 2), 1.0 / math.sqrt(hd), ctx)
             o = o.transpose(1, 2).reshape(B, 1, nh * hd)
             h, x = ops.rmsnorm(h, n2.weight, n2.variance_epsilon, residual=a.o_proj(o))
             gate, up = self._parallel(x, [mlp.gate_proj, mlp.up_proj])
@@ -143,9 +158,9 @@ class GraphDecoder:
     def _layers_llama(self, h):
         B, nh, nkv, hd = self.batch, self.nh, self.nkv, self.hd
         pos = self.position
-        cos = self.cos.index_select(0, pos)[None, None]                                    # (1, 1, 1, hd)
-        sin = self.sin.index_select(0, pos)[None, None]
-        mask = (self._arange <= pos)[None, None, None, :]                                  # (1, 1, 1, max_len)
+        cos = self.cos.index_select(0, pos).view(-1, 1, 1, hd)                             # (1 or B, 1, 1, hd)
+        sin = self.sin.index_select(0, pos).view(-1, 1, 1, hd)
+        ctx = self._attn_context()
         for li, layer in enumerate(self.layers):
             a = layer.self_attn
             x = layer.input_layernorm(h)
@@ -155,13 +170,7 @@ class GraphDecoder:
             v = v.view(B, 1, nkv, hd).transpose(1, 2)
             q = q * cos + _rotate_half(q) * sin
             k = k * cos + _rotate_half(k) * sin
-            self.k_cache[li].index_copy_(2, pos, k)
-            self.v_cache[li].index_copy_(2, pos, v)
-            kk, vv = self.k_cache[li], self.v_cache[li]
-            if nkv != nh:
-                kk = kk.repeat_interleave(nh // nkv, dim=1)
-                vv = vv.repeat_interleave(nh // nkv, dim=1)
-            o = F.scaled_dot_product_attention(q, kk, vv, attn_mask=mask, scale=1.0 / math.sqrt(hd))
+            o = self._attend(li, q, k, v, 1.0 / math.sqrt(hd), ctx)
             o = o.transpose(1, 2).reshape(B, 1, nh * hd)
             h = h + a.o_proj(o)
             x = layer.post_attention_layernorm(h)
@@ -174,16 +183,13 @@ class GraphDecoder:
     # biases live inside the (Quant)Linear modules
     def _layers_opt(self, h):
         B, nh, hd = self.batch, self.nh, self.hd
-        pos = self.position
-        mask = (self._arange <= pos)[None, None, None, :]
+        ctx = self._attn_context()
         for li, layer in enumerate(self.layers):
             a, before = layer.self_attn, layer.do_layer_norm_before
             x = layer.self_attn_layer_norm(h) if before else h
             q, k, v = self._parallel(x, [a.q_proj, a.k_proj, a.v_proj])
             q = (q * a.scaling).view(B, 1, nh, hd).transpose(1, 2)                         # scaled first, as the HF module does
-            self.k_cache[li].index_copy_(2, pos, k.view(B, 1, nh, hd).transpose(1, 2))
-            self.v_cache[li].index_copy_(2, pos, v.view(B, 1, nh, hd).transpose(1, 2))
-            o = F.scaled_dot_product_attention(q, self.k_cache[li], self.v_cache[li], attn_mask=mask, scale=1.0)
+            o = self._attend(li, q, k.view(B, 1, nh, hd).transpose(1, 2), v.view(B, 1, nh, hd).transpose(1, 2), 1.0, ctx)
             h = h + a.out_proj(o.transpose(1, 2).reshape(B, 1, nh * hd))
             if not before:
                 h = layer.self_attn_layer_norm(h)
@@ -201,7 +207,7 @@ class GraphDecoder:
         h = d.embed_tokens(self.tokens)[:, None, :]
         if d.project_in is not None:
             h = d.project_in(h)
-        return h + F.embedding(self.position + d.embed_positions.offset, d.embed_positions.weight)[None]
+        return h + F.embedding(self.position + d.embed_positions.offset, d.embed_positions.weight)[:, None]
 
     def _head(self, h, pend):
         """Final norm (fused with the pending residual add on the glue-kernel path) -> lm_head: logits (B, vocab)."""
@@ -248,6 +254,8 @@ class GraphDecoder:
                 self._step()
             self.position.copy_(pos0)
             self.graph = torch.cuda.CUDAGraph()
+            for gen in self._graph_generators():
+                self.graph.register_generator_state(gen)
             with torch.cuda.graph(self.graph, stream=side, capture_error_mode='thread_local'):
                 self._step()
         torch.cuda.current_stream(self.dev).wait_stream(side)
